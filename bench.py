@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — Mpps of the subscriber-dataplane hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload pipeline_imix] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload pipeline_imix] [--impl reference] [--dump-outputs DIR]
 
 A *step* is one batch of 2^22 synthetic frames per GPU through the program of
 the chosen workload (default: the full pipeline antispoof -> NAT44 -> QoS on
@@ -288,10 +288,51 @@ def _traffic(name, kernel, world, reference_capacities):
     return ent, "profiles/ncu_traffic.json"
 
 
-def measure(a, name, frames, steps, warmup, *, wl=None, reference_capacities=False, subs_scale=1, keep=False):
+# --dump-outputs writes at most 36 + 2 x 12 MiB (under 64 MB).  The frame sample depends on the batch alone, not on
+# what a build emitted, so two builds dump the same frames.
+DUMP_FRAME_BYTES = 36 << 20  # frames, verdicts, lengths and frame indices
+DUMP_EVENT_BYTES = 12 << 20  # records of one event ring
+
+
+def dump_outputs(out_dir, n, hw, arena_d, off_d, stride, len_d, verdict_d, events):
+    """What the last timed step handed back, as DIR/<name>.npy: verdict, len and the first `hw` bytes of every frame
+    (the bytes the step restored and the program may rewrite), as float32, and the frames' indices (frame_index,
+    float64); above DUMP_FRAME_BYTES a fixed seeded sample of frames (sorted) stands for the batch.  And the records
+    the step emitted into each event ring (`events`: ring -> u8[records, size], drained after the step), as float32
+    bytes with the padding the reference leaves uninitialised zeroed (ev_<ring>: the first DUMP_EVENT_BYTES of them in
+    ring order; no file for a ring the step left empty)."""
+    import torch
+    from bng_b200.layouts import PADDING
+    outs = {}
+    for ring, rec in events.items():
+        if rec.shape[0] == 0:
+            continue
+        rec = rec[: DUMP_EVENT_BYTES // (4 * rec.shape[1])].copy()
+        for off, ln in PADDING.get(ring, ()):
+            rec[:, off:off + ln] = 0
+        outs["ev_" + ring] = rec.astype(np.float32)
+    per_frame = (hw + 2) * 4 + 8
+    if n * per_frame <= DUMP_FRAME_BYTES:
+        idx = np.arange(n, dtype=np.int64)
+    else:
+        idx = np.sort(np.random.default_rng(0xB200).choice(n, DUMP_FRAME_BYTES // per_frame, replace=False))
+    idx_d = torch.from_numpy(idx).to(arena_d.device)
+    if off_d is None:
+        frames = arena_d[: n * stride].view(n, stride)[idx_d, :hw]
+    else:
+        frames = arena_d[off_d.long()[idx_d, None] * 16 + torch.arange(hw, device=arena_d.device)[None, :]]
+    os.makedirs(out_dir, exist_ok=True)
+    outs.update({"frame_index": idx.astype(np.float64), "verdict": verdict_d[idx_d].cpu().numpy().astype(np.float32),
+                 "len": len_d[idx_d].cpu().numpy().astype(np.float32), "frames": frames.cpu().numpy().astype(np.float32)})
+    for k, v in outs.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
+def measure(a, name, frames, steps, warmup, *, wl=None, reference_capacities=False, subs_scale=1, keep=False, dump=None):
     """One workload on this rank's GPU: W warm-up steps, K timed steps (CUDA events on the library's stream, fresh
     frames restored untimed between steps), max over ranks, then a per-kernel pass for the roofline.  Returns the
-    result dict; with keep=True also the live objects the end-to-end leg needs."""
+    result dict; with keep=True also the live objects the end-to-end leg needs; with dump=DIR the outputs of the last
+    timed step are written there (dump_outputs)."""
     import torch
     from bng_b200 import MEM_DEVICE, Dataplane
     from bng_b200.layouts import as_bytes
@@ -391,6 +432,9 @@ def measure(a, name, frames, steps, warmup, *, wl=None, reference_capacities=Fal
     clocks = sampler.result()
     drops = int((verdict_d == 2).sum().item())
     value = frames_all * steps / (total_ms_max * 1e-3) / 1e6
+    if dump:  # before the per-kernel pass below overwrites the arena
+        dump_outputs(dump, n, hw, arena_d, off_d, stride, len_d, verdict_d,
+                     {ring: dp.drain(ring) for ring in ("spoof_events", "nat_log_rb")})
 
     # ---- per-kernel timing for the roofline (separate pass, events around every launch) ----
     dp.prof_enable(True)
@@ -593,7 +637,9 @@ def run_gpu(a):
     t_start = time.time()
 
     # ---- headline: the workload at BASELINE's population, tables sized for it ----
-    head, live = measure(a, a.workload, a.frames, a.steps, a.warmup, reference_capacities=a.reference_capacities, keep=True)
+    dump = a.dump_outputs and (a.dump_outputs if world == 1 else os.path.join(a.dump_outputs, f"rank{rank}"))
+    head, live = measure(a, a.workload, a.frames, a.steps, a.warmup, reference_capacities=a.reference_capacities, keep=True,
+                         dump=dump)
     wl, dp = live["wl"], live["dp"]
     e2e, e2e_extra = e2e_leg(a, live) if a.e2e_steps > 0 else (None, None)  # 0: kernel-only runs under a profiler
 
@@ -714,7 +760,7 @@ def run_dhcp_slow(a):
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     import test_host_mirror
     test_host_mirror.build_host_test()
-    rounds = max(1, a.steps) * 100
+    rounds = a.steps  # one step = one round of 1 000 DISCOVERs
     j = json.loads(subprocess.run([test_host_mirror.SLOW_BIN, str(rounds)], capture_output=True, text=True, check=True).stdout)
     print(json.dumps({
         "metric": "DHCP DISCOVER/s (slow path, CPU only)", "value": round(j["req_per_s"], 1), "unit": "requests/s", "n_gpus": 0,
@@ -732,8 +778,12 @@ def run_dhcp_slow(a):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of the headline, of --impl reference and of dhcp_slow (1 000 DISCOVERs each).  The "
+                         "side measurements of the GPU arm keep their own counts: the end-to-end leg min(K, --e2e-steps), "
+                         "the reference-capacities and per-GPU-constant variants min(max(K, 3), 10), the other "
+                         "workloads 5, the one-core CPU baseline 20 passes")
+    ap.add_argument("--warmup", type=int, default=3, help="untimed steps before the timed ones (at least 3 on the GPU)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="pipeline_imix", choices=sorted(W.BUILDERS) + ["dhcp_slow"],
                     help="dhcp_slow = BASELINE config #1: the DHCP slow path (CPU only, plumbing; no GPU involved)")
@@ -748,7 +798,15 @@ def main():
                     help="diagnostic: run ONE GPU as shard R of an N-GPU job (its subscribers, its frames) without the other ranks")
     ap.add_argument("--no-extra", action="store_true",
                     help="only the headline: skip the reference-capacities variant, the per-GPU-constant variant and the other configs")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the headline's last timed step computed (verdicts, lengths, frame bytes, event "
+                         "records; a fixed sample of frames above 36 MiB) to DIR/<name>.npy as float32, to "
+                         "compare two builds")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "ours" or a.workload == "dhcp_slow"):
+        ap.error("--dump-outputs writes the outputs of the GPU arm")
     a.warmup = max(a.warmup, 3) if a.impl == "ours" else a.warmup
     if a.as_shard:
         G.as_shard = tuple(int(x) for x in a.as_shard.split("/"))

@@ -9,6 +9,8 @@ asserts two result sets are bit-identical (compiler padding masked).
 """
 from __future__ import annotations
 
+import hashlib
+
 import numpy as np
 
 from bng_b200 import layouts as L
@@ -292,3 +294,26 @@ def save_golden(path: str, res: dict):
 def load_golden(path: str) -> dict:
     with np.load(path) as z:
         return {k: z[k] for k in z.files}
+
+
+def fingerprint(res: dict) -> dict:
+    """Per result key: the array's shape and the SHA-256 of its bytes (first 64 bits), or "empty" for an array with
+    no rows, as diff_keys treats those.  Lets a result set too large to store be pinned bit for bit."""
+    out = {}
+    for k, v in res.items():
+        a = np.ascontiguousarray(v)
+        if a.shape[0] == 0:
+            out[k] = "empty"
+        else:
+            out[k] = "x".join(map(str, a.shape)) + ":" + hashlib.sha256(a.tobytes()).hexdigest()[:16]
+    return out
+
+
+def compare_fingerprint(want: dict, res: dict, what: str = ""):
+    """compare() against a stored fingerprint(): lists every result key whose shape or bytes differ."""
+    got = fingerprint(res)
+    diffs = [(k, "present on one side only") for k in sorted(set(want) ^ set(got))]
+    diffs += [(k, f"{want[k]} vs {got[k]}") for k in sorted(set(want) & set(got)) if want[k] != got[k]]
+    if diffs:
+        lines = "\n".join(f"  {k}: {msg}" for k, msg in diffs[:40])
+        raise AssertionError(f"{what}: {len(diffs)} result keys differ (shape:sha256)\n{lines}")
